@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""bench.py -- headline benchmark of the two DetectorFreeSfM hot paths on B200 (contract: task statement / DESIGN.md).
+"""bench.py -- headline benchmark of the two DetectorFreeSfM hot paths on B200 (DESIGN.md).
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the reference's CPU path: the oracle port, bounded sample)
+  python bench.py ... --dump-outputs DIR                   (also write what the last timed step of every leg returned, as .npy)
 
 One "step" = one pass of HP-1 over the demo-scene workload C2: 8 synthetic 832x832 images, exhaustive pairing = 28 image
 pairs, each pair -> (M,5) matches (BASELINE.json configs[1]).  `value` = image-pairs/s with the images resident in HBM and
@@ -99,6 +100,24 @@ def measured_peaks():
             d = json.load(f)
         return {"tflops": d["bf16_tflops_sustained"], "hbm": d["hbm_gbs"], "src": "measured (MEASURED_PEAKS.json, sustained bf16)"}
     return {"tflops": 1590.0, "hbm": 6650.0, "src": "fallback (B200_PROFILING.md)"}
+
+
+DUMP_MAX_ELEMS = 1 << 20      # per array; the at most 16 arrays written stay under 64 MB in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float32 (float64 for integer arrays, exact below 2^53).  An array of more than
+    DUMP_MAX_ELEMS elements is replaced by a fixed, seeded sample of its flattened elements (sorted indices), so that two builds
+    given the same arguments can be compared file by file."""
+    assert len(arrays) <= 16
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64)
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def profile_report(lib):
@@ -335,7 +354,16 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-post", action="store_true")
     ap.add_argument("--skip-img", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each leg returned as DIR/<name>.npy (float32 / float64; "
+                         "arrays over 2^20 elements as a fixed seeded sample): hp1_* the per-pair matches and their keypoint merge, hp2_* "
+                         "the refined chunk, post_* the keypoint merge, image_* the resized images; rank 0 only.  bench_outputs/ in "
+                         "the repository is git-ignored for this")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "c2"):
+        ap.error("--dump-outputs writes the outputs of the default workload (--impl b200 --config c2)")
     if args.impl == "reference":
         return run_reference(args)
     if args.config == "c4":
@@ -351,7 +379,8 @@ def main():
     dev = torch.device("cuda", local)
     lib = _lib.load_library()
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
+    outputs = {}      # --dump-outputs: name -> host array of the last timed step
 
     # ------------------------------------------------------------------ HP-1 workload: one scene per rank
     matcher = B200LoFTR(util.loftr_config(thr=0.2, temperature=0.1), feature_cache_size=2 * N_IMAGES).cuda(local).eval()
@@ -467,6 +496,7 @@ def main():
         return res
 
     def timed(fn, steps, gather):
+        """-> (max over ranks of the ms the steps took, what the last step returned)"""
         D.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -478,7 +508,7 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         D.barrier()
-        return D.max_over_ranks(e0.elapsed_time(e1), dev)
+        return D.max_over_ranks(e0.elapsed_time(e1), dev), out
 
     for _ in range(W):
         warm = step_resident(False)
@@ -489,21 +519,26 @@ def main():
         sampler.start()
         time.sleep(0.3)
     launches0 = lib.dfsfm_launch_count()
-    ms_cold = timed(lambda: step_resident(False), K, True)
+    ms_cold, last = timed(lambda: step_resident(False), K, True)
     launches = lib.dfsfm_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        kp, score, img_off, ids = m_stats["merged"]
+        outputs.update(hp1_matches=torch.cat(last, 0), hp1_match_counts=torch.tensor([o.shape[0] for o in last]), hp1_keypoints=kp,
+                       hp1_keypoint_scores=score, hp1_image_keypoint_offsets=img_off, hp1_match_keypoint_ids=ids)
+        outputs = {k: v.cpu() for k, v in outputs.items()}
     ms_cold_1w = None
     if n_workers > 1:     # the same step with ONE pair in flight (per-pair latency view; explains what the pair workers buy)
         saved_w, n_workers = n_workers, 1
         step_resident(False)
-        ms_cold_1w = timed(lambda: step_resident(False), K, False)
+        ms_cold_1w, _ = timed(lambda: step_resident(False), K, False)
         n_workers = saved_w
     step_resident(True)   # every variant gets its own untimed warm-up step (allocator growth, feature-cache storage)
-    ms_cached = timed(lambda: step_resident(True), K, True)
+    ms_cached, _ = timed(lambda: step_resident(True), K, True)
     step_e2e(False)
-    ms_e2e = timed(lambda: step_e2e(False), K, True)
+    ms_e2e, _ = timed(lambda: step_e2e(False), K, True)
     step_e2e(True)
-    ms_e2e_cached = timed(lambda: step_e2e(True), K, True)
+    ms_e2e_cached, _ = timed(lambda: step_e2e(True), K, True)
     n_pairs = len(pairs) * world
 
     # ------------------------------------------------------------------ roofline attribution of the dominant kernel
@@ -579,9 +614,11 @@ def main():
 
         for _ in range(2):
             chunk_resident()
-        k2 = max(2, min(K, 3))
-        ms2 = timed(chunk_resident, k2, False)
-        ms2_e2e = timed(chunk_e2e, k2, False)
+        ms2, last = timed(chunk_resident, K, False)
+        if args.dump_outputs:
+            outputs.update(hp2_query_points_refined=last["query_points_refined"].cpu(),
+                           hp2_reference_points_refined=last["reference_points_refined"][-1].cpu(), hp2_std=last["std"][-1].cpu())
+        ms2_e2e, _ = timed(chunk_e2e, K, False)
         lib.dfsfm_profile_enable(1)
         chunk_resident()
         prof2 = profile_report(lib)
@@ -590,9 +627,9 @@ def main():
         # algorithmic FLOPs per patch of the GEMM convolutions as the reference executes them (SURVEY 8d: 1.024 GFLOP/patch
         # incl. the 4.2 MFLOP conv1_1 which is a SIMT kernel here)
         pconv_alg = n_patches * (1.024e9 - 2 * 35 * 35 * 27 * 64)
-        hp2 = {"metric": "tracks/s refinement", "value": args.hp2_tracks * k2 * world / (ms2 * 1e-3), "unit": "tracks/s",
-               "ms_per_chunk": ms2 / k2, "tracks_per_chunk": args.hp2_tracks, "patches_per_chunk": n_patches,
-               "e2e": {"value": args.hp2_tracks * k2 * world / (ms2_e2e * 1e-3), "unit": "tracks/s",
+        hp2 = {"metric": "tracks/s refinement", "value": args.hp2_tracks * K * world / (ms2 * 1e-3), "unit": "tracks/s",
+               "ms_per_chunk": ms2 / K, "tracks_per_chunk": args.hp2_tracks, "patches_per_chunk": n_patches,
+               "e2e": {"value": args.hp2_tracks * K * world / (ms2_e2e * 1e-3), "unit": "tracks/s",
                        "h2d_bytes_per_step": h2d_2, "d2h_bytes_per_step": d2h_2,
                        "note": "host chunk dict (pinned) -> device, matcher call, refined points + std -> host; inside the call the shim reads the "
                                "small per-track arrays back ONCE as one packed buffer (the C ABI builds its patch records on the host; ~0.5 MB, "
@@ -630,18 +667,20 @@ def main():
 
             for _ in range(2):
                 post_resident()
-            k3 = max(2, min(K, 3))
-            ms3 = timed(post_resident, k3, False)
-            ms3_e2e = timed(post_e2e, k3, False)
+            ms3, last = timed(post_resident, K, False)
+            if args.dump_outputs:
+                outputs.update({"post_" + n: t.cpu() for n, t in zip(("keypoints", "keypoint_scores", "image_keypoint_offsets",
+                                                                       "match_keypoint_ids"), last)})
+            ms3_e2e, _ = timed(post_e2e, K, False)
             lib.dfsfm_profile_enable(1)
             kp = post_resident()
             prof3 = profile_report(lib)
             lib.dfsfm_profile_enable(0)
             sc_cnt, sc_ms = prof3.get("post_scatter", (0, 0.0))
             rec_bytes = 24.0 * n_obs   # one pass streams every 12-byte (key, value) record in and out once
-            post = {"metric": "match end points/s merged into key points", "value": n_obs * k3 * world / (ms3 * 1e-3), "unit": "observations/s",
-                    "ms_per_call": ms3 / k3, "observations": n_obs, "pairs": len(pairs), "images": n_img, "keypoints": int(kp[0].shape[0]),
-                    "e2e": {"value": n_obs * k3 * world / (ms3_e2e * 1e-3), "unit": "observations/s", "h2d_bytes_per_step": rows_host.numel() * 4,
+            post = {"metric": "match end points/s merged into key points", "value": n_obs * K * world / (ms3 * 1e-3), "unit": "observations/s",
+                    "ms_per_call": ms3 / K, "observations": n_obs, "pairs": len(pairs), "images": n_img, "keypoints": int(kp[0].shape[0]),
+                    "e2e": {"value": n_obs * K * world / (ms3_e2e * 1e-3), "unit": "observations/s", "h2d_bytes_per_step": rows_host.numel() * 4,
                             "d2h_bytes_per_step": int(kp[0].numel() * 4 + kp[1].numel() * 4 + kp[3].numel() * 4)},
                     "roofline": {"bound": "hbm", "kernel": "rs_scatter_kernel (one 8-bit LSD radix pass over the observation records)",
                                  "achieved": rec_bytes / (sc_ms / sc_cnt * 1e-3) / 1e9 if sc_cnt else None, "peak": peaks.get("hbm"), "unit": "GB/s",
@@ -687,18 +726,19 @@ def main():
 
             for _ in range(2):
                 img_resident()
-            k4 = max(2, min(K, 3))
-            ms4 = timed(img_resident, k4, False)
-            ms4_e2e = timed(img_e2e, k4, False)
+            ms4, last = timed(img_resident, K, False)
+            if args.dump_outputs:
+                outputs["image_resized"] = torch.stack(last, 0).cpu()
+            ms4_e2e, _ = timed(img_e2e, K, False)
             lib.dfsfm_profile_enable(1)
             img_resident()
             prof4 = profile_report(lib)
             lib.dfsfm_profile_enable(0)
             h_cnt, h_ms = prof4.get("resize_h", (0, 0.0))
             alg_bytes = float(src_hw[0] * src_hw[1] + src_hw[0] * size[0])      # horizontal pass: bytes in + intermediate bytes out
-            img_leg = {"metric": "images/s resized (12 MP gray -> longest side 1200, PIL-LANCZOS parity) + /255", "value": n_img * k4 * world / (ms4 * 1e-3),
-                       "unit": "images/s", "ms_per_image": ms4 / (k4 * n_img), "src_hw": list(src_hw), "out_wh": list(size),
-                       "e2e": {"value": n_img * k4 * world / (ms4_e2e * 1e-3), "unit": "images/s", "h2d_bytes_per_step": n_img * photo.size,
+            img_leg = {"metric": "images/s resized (12 MP gray -> longest side 1200, PIL-LANCZOS parity) + /255", "value": n_img * K * world / (ms4 * 1e-3),
+                       "unit": "images/s", "ms_per_image": ms4 / (K * n_img), "src_hw": list(src_hw), "out_wh": list(size),
+                       "e2e": {"value": n_img * K * world / (ms4_e2e * 1e-3), "unit": "images/s", "h2d_bytes_per_step": n_img * photo.size,
                                "d2h_bytes_per_step": 0},
                        "roofline": {"bound": "hbm", "kernel": "lanczos_h_kernel (horizontal pass over the full-resolution image)",
                                     "achieved": alg_bytes / (h_ms / h_cnt * 1e-3) / 1e9 if h_cnt else None, "peak": peaks["hbm"], "unit": "GB/s",
@@ -754,6 +794,8 @@ def main():
             "gpu_launches": total_launches, "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu,
             "algorithmic_gflop_per_pair": pair_flops(HW, HW) / 1e9, "hp2": hp2, "post": post, "image_pipeline": img_leg,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         torch.distributed.destroy_process_group()

@@ -1,5 +1,6 @@
-"""Generate the committed golden fixtures by running the UNMODIFIED reference modules (imported from /root/reference via
-oracle/ref_shims.py) on seeded inputs.  Build-container only.  Usage:  python tests/golden/make_golden.py
+"""Generate the committed golden fixtures by running the UNMODIFIED reference modules (imported from the reference tree via
+oracle/ref_shims.py) on seeded inputs.  Needs the reference tree (oracle/ref_shims.py: DFSFM_REFERENCE).
+Usage:  python tests/golden/make_golden.py [chunk_dataset | reference_outputs | chunk_dataset_cases ...]   (no argument: all)
 
 Fixtures (small, fp32, torch.save):
   roialign_readme.pt   the reference's own known-answer vector (third_party/RoIAlign.pytorch/README.md:42-96)
@@ -8,6 +9,10 @@ Fixtures (small, fp32, torch.save):
   postprocess_small.pt Match2Kpts + keypoint_worker + update_matches + transform_keypoints on synthetic matches of 5 images
   refine_worker_small.pt  matchWorker (the reference's refinement host loop) on three small chunks with a stand-in matcher
   image_small.pt       read_grayscale (cv2 decode of a PNG written here, PIL-LANCZOS resize, /255) on three synthetic images
+  reference_outputs.pt what tests/test_oracle_vs_reference.py compares the oracle with: LoFTR coarse + fine and MultiviewMatcher
+                       whole, RoIAlign C++ as a seeded sample + sums, post-processing and read_grayscale images as checksums
+  chunk_dataset_cases.pt  MatchingMultiviewData on the four cases of tests/test_chunk_dataset_cpu.py (bags and every chunk dict
+                       as checksums) + CoarseColmapDataset.update_refined_kpts_to_colmap_multiview on one write-back case
 """
 import os
 import sys
@@ -145,6 +150,115 @@ def postprocess_golden():
     return {"names": names, "matches": matches, "final_keypoints": fk, "final_scores": fs, "updated_matches": upd}
 
 
+LOFTR_CASE = {"hw": (64, 96), "seed": 3, "scale0": [[1.5, 1.25]], "scale1": [[1.0, 2.0]], "thr": 0.0, "temperature": 0.01}
+MULTIVIEW_CASE = {"M": 20, "n_img": 4, "max_views": 3, "seed": 9}
+POSTPROCESS_CASES = [(4, 50), (6, 300), (5, [0, 10, 200]), (3, 1)]
+IMAGE_CASES = [(150, 200, (96,), 8), (97, 61, (128,), 8), (64, 80, None, None), (300, 200, (64, 48), None)]
+
+
+def loftr_case_input():
+    im0, im1 = util.synth_pair(*LOFTR_CASE["hw"], seed=LOFTR_CASE["seed"])
+    return {"image0": im0, "image1": im1, "scale0": torch.tensor(LOFTR_CASE["scale0"]), "scale1": torch.tensor(LOFTR_CASE["scale1"])}
+
+
+def roialign_case_input():
+    """image [2,3,40,56], 64 boxes (normalised, partly outside the image), box indices"""
+    g = torch.Generator().manual_seed(0)
+    image = torch.rand(2, 3, 40, 56, generator=g)
+    nb = torch.rand(64, 4, generator=g) * 1.4 - 0.2
+    nb[:, 2:] = nb[:, :2] + torch.rand(64, 2, generator=g) * 0.6
+    bi = torch.randint(0, 2, (64,), generator=g, dtype=torch.int32)
+    return image, nb.contiguous(), bi
+
+
+def postprocess_case_input(seed):
+    import itertools
+    n, m = POSTPROCESS_CASES[seed]
+    pairs = list(itertools.combinations(range(n), 2))
+    if seed == 2:
+        pairs = [p for p in pairs if 4 not in p]    # image 4 never matched
+    return util.synth_matches(n, pairs, m, seed=seed)
+
+
+def sample_of(t, n=4096):
+    """a fixed, seeded sample of a tensor too large to store whole: flat indices, their values, float64 sum and abs-sum"""
+    f = t.flatten()
+    idx = torch.randperm(f.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+    return {"shape": list(t.shape), "idx": idx, "values": f[idx].clone(), "sum": f.double().sum().item(), "abs_sum": f.double().abs().sum().item()}
+
+
+def reference_outputs():
+    """the reference's own outputs on the inputs tests/test_oracle_vs_reference.py gives the oracle"""
+    out = {"loftr": {}}
+    LoFTR, _ = ref_shims.import_loftr()
+    sd = weights.loftr_state_dict(0)
+    for fine in (False, True):
+        m = LoFTR(ref_shims.loftr_config(thr=LOFTR_CASE["thr"], fine=fine, temperature=LOFTR_CASE["temperature"])).eval()
+        m.load_state_dict(sd, strict=True)
+        d = loftr_case_input()
+        with torch.no_grad():
+            m(d)
+        out["loftr"][fine] = {k: d[k] for k in ("conf_matrix", "i_ids", "j_ids", "mconf", "mkpts0_f", "mkpts1_f")}
+    MM = ref_shims.import_multiview()
+    m = MM(config=ref_shims.multiview_config(15, 7), test=True).eval()
+    m.load_state_dict(weights.multiview_state_dict(0), strict=True)
+    d = util.synth_chunk(**MULTIVIEW_CASE)
+    with torch.no_grad():
+        m(d)
+    out["multiview"] = {"query_points_refined": d["query_points_refined"], "reference_points_refined": d["reference_points_refined"][-1],
+                        "std": d["std"][-1]}
+    ext = ref_shims.build_ref_roialign()
+    image, boxes, box_index = roialign_case_input()
+    crops = torch.zeros(1)
+    ext.forward(image, boxes, box_index, 0.0, 35, 35, crops)
+    out["roialign"] = sample_of(crops)
+    out["postprocess"] = [tuple({k: checksum(a) for k, a in part.items()} for part in reference_postprocess(*postprocess_case_input(seed)))
+                          for seed in range(len(POSTPROCESS_CASES))]
+    import tempfile
+    out["image"] = []
+    with tempfile.TemporaryDirectory() as tmp:
+        for seed, (h, w, resize, df) in enumerate(IMAGE_CASES):
+            t, scales, hw = reference_read_grayscale(util.synth_photo(h, w, seed), resize, df, tmp)
+            out["image"].append((checksum(t), scales, hw))
+    return out
+
+
+def checksum(t):
+    """order-sensitive checksum of a tensor or numpy array: shape, dtype, float64 sum and position-weighted sum"""
+    f = torch.as_tensor(t).flatten().double()
+    return {"shape": list(t.shape), "dtype": str(t.dtype), "sum": f.sum().item(),
+            "wsum": (f * torch.arange(1, f.numel() + 1, dtype=torch.float64)).sum().item()}
+
+
+def checksum_close(t, want, rel=1e-12):
+    """``t`` against a stored checksum(): same shape and dtype, both sums equal to within rel * (|t_i| + 1) per element -- with the
+    default, equal up to float64 summation order"""
+    got = checksum(t)
+    f = torch.as_tensor(t).flatten().double().abs()
+    pos = torch.arange(1, f.numel() + 1, dtype=torch.float64)
+    return (got["shape"] == want["shape"] and got["dtype"] == want["dtype"]
+            and abs(got["sum"] - want["sum"]) <= rel * (f.sum().item() + f.numel())
+            and abs(got["wsum"] - want["wsum"]) <= rel * ((f * pos).sum().item() + pos.sum().item()))
+
+
+def chunk_dataset_cases():
+    """the reference's MatchingMultiviewData on every case of tests/test_chunk_dataset_cpu.py (the bags and every chunk dict as
+    checksums: the whole items would be several MB) and its update_refined_kpts_to_colmap_multiview on write-back case 5"""
+    import types
+    from tests.test_chunk_dataset_cpu import CASES, _case_args, _writeback_case, _flat_bags
+    Ref = ref_shims.import_chunk_dataset()
+    cases = []
+    for case in range(len(CASES)):
+        ds, cfg, split = _case_args(case)
+        ref = Ref(ds, cfg, worker_split_idxs=split)
+        cases.append({"case": CASES[case], "bags": checksum(_flat_bags(ref.image_bags)),
+                      "items": [{k: (len(v) if k == "images" else checksum(v)) for k, v in ref[i].items()} for i in range(len(ref))]})
+    a, _, results = _writeback_case(5)
+    ref_cls = ref_shims.import_colmap_dataset_class()
+    ref_cls.update_refined_kpts_to_colmap_multiview(types.SimpleNamespace(colmap_images=a), results)
+    return {"cases": cases, "writeback": {c: a[c].xys for c in a}}
+
+
 def chunk_dataset_golden():
     """the reference's own MatchingMultiviewData (bags + every chunk dict) on one synthetic COLMAP model"""
     Ref = ref_shims.import_chunk_dataset()
@@ -156,9 +270,12 @@ def chunk_dataset_golden():
     return {"case": case, "cfg": cfg, "bags": bags, "items": [{k: v for k, v in ref[i].items() if k != "images"} for i in range(len(ref))]}   # images: pass-through of ds[...]
 
 
+PARTS = {"chunk_dataset": (chunk_dataset_golden, "chunk_dataset_small.pt"), "reference_outputs": (reference_outputs, "reference_outputs.pt"),
+         "chunk_dataset_cases": (chunk_dataset_cases, "chunk_dataset_cases.pt")}
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "chunk_dataset":
-        torch.save(chunk_dataset_golden(), os.path.join(HERE, "chunk_dataset_small.pt"))
-    else:
+    if len(sys.argv) == 1:
         main()
-        torch.save(chunk_dataset_golden(), os.path.join(HERE, "chunk_dataset_small.pt"))
+    for part in sys.argv[1:] or list(PARTS):
+        fn, name = PARTS[part]
+        torch.save(fn(), os.path.join(HERE, name))

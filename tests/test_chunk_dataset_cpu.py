@@ -1,6 +1,6 @@
 """SURVEY 8(f) row 2 / 8(a) row b2 on the CPU box: the native bag assignment + chunk dataset against (i) the running CPython's set
-semantics (the order the reference's greedy loop depends on) and (ii) the reference's own MatchingMultiviewData class imported from
-/root/reference on synthetic COLMAP models (skipped on the GPU box, where that tree does not exist: a stored golden covers it there)."""
+semantics (the order the reference's greedy loop depends on) and (ii) what the reference's own MatchingMultiviewData class produced
+on synthetic COLMAP models (stored under tests/golden by tests/golden/make_golden.py)."""
 import ctypes
 import os
 import random
@@ -10,10 +10,10 @@ import pytest
 import torch
 
 from detectorfreesfm_b200 import _lib
-from oracle import ref_shims
 from tests import util
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "chunk_dataset_small.pt")
+CASES_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "chunk_dataset_cases.pt")
 
 
 def _pyset(lib, op, a, b):
@@ -61,20 +61,43 @@ CASES = [dict(n_images=6, n_points=60, max_obs=5, seed=1), dict(n_images=12, n_p
          dict(n_images=30, n_points=900, max_obs=25, seed=3, dup_frac=0.1), dict(n_images=40, n_points=1500, max_obs=12, seed=4, first_image_id=900)]
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference not present")
-@pytest.mark.parametrize("case", range(len(CASES)))
-def test_bags_and_chunks_match_reference_class(case):
-    from detectorfreesfm_b200.chunk_dataset import B200MatchingMultiviewData
-    Ref = ref_shims.import_chunk_dataset()
+def _case_args(case):
+    """-> (dataset, cfg, worker_split_idxs) of CASES[case]"""
     ds = util.SynthColmapDataset(**CASES[case])
     cfg = {"max_track_length": 16, "chunk": 50 if case != 1 else 2000}
     split = None if case != 3 else list(range(0, len(ds.colmap_3ds), 2))[::-1]      # a worker's share, in its own order
-    ref = Ref(ds, cfg, worker_split_idxs=split)
+    return ds, cfg, split
+
+
+def _flat_bags(bags):
+    """the bags as one int64 sequence: per bag its image ids, track ids and (reference image, query images) per track, each list
+    preceded by its length"""
+    flat = []
+    for b in _as_lists(bags):
+        flat += [len(b["bag_image_ids"])] + b["bag_image_ids"] + [len(b["track_ids"])] + b["track_ids"]
+        for ref_img, q in b["track_corresponding_imgs"]:
+            flat += [ref_img, len(q)] + q
+    return torch.tensor(flat, dtype=torch.int64)
+
+
+@pytest.mark.parametrize("case", range(len(CASES)))
+def test_bags_and_chunks_match_reference_class(case):
+    """bags and every chunk dict vs the reference class's, stored as checksums (tests/golden/chunk_dataset_cases.pt): equal shapes,
+    dtypes and values up to float64 summation order, the float64 geometry within rtol = atol = 1e-9"""
+    from detectorfreesfm_b200.chunk_dataset import B200MatchingMultiviewData
+    from tests.golden.make_golden import checksum_close
+    g = torch.load(CASES_GOLDEN, weights_only=False)["cases"][case]
+    assert g["case"] == CASES[case]
+    ds, cfg, split = _case_args(case)
     ours = B200MatchingMultiviewData(ds, cfg, worker_split_idxs=split)
-    assert _as_lists(ours.image_bags) == _as_lists(ref.image_bags)
-    assert len(ours) == len(ref) and (len(ref) > 1 or case == 1)
-    for i in range(len(ref)):
-        _compare_items(ours[i], ref[i])
+    assert checksum_close(_flat_bags(ours.image_bags), g["bags"])
+    assert len(ours) == len(g["items"]) and (len(ours) > 1 or case == 1)
+    for i, want in enumerate(g["items"]):
+        item = ours[i]
+        assert set(item.keys()) == set(want.keys())
+        assert len(item.pop("images")) == want["images"]
+        for k, v in item.items():
+            assert checksum_close(v, want[k], 1e-9 if k in ("scales_relative", "view_point_vector") else 1e-12), (i, k)
     # every query node of every assigned track lands in exactly one chunk
     total = sum(int(ours[i]["track_valid_mask"].sum()) for i in range(len(ours)))
     want = sum(len(set(ds.colmap_3ds[t].image_ids.tolist()) - {int(ours.point3d_assignment[t][0])}) for t in ours.point3d_assignment)
@@ -122,12 +145,10 @@ def test_colmap_writeback_matches_the_reference_loop():
         assert all(np.array_equal(a[c].xys, b[c].xys) for c in a)
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference not present")
 def test_colmap_writeback_matches_the_reference_method():
-    import types
+    """vs the key points CoarseColmapDataset.update_refined_kpts_to_colmap_multiview wrote (tests/golden/chunk_dataset_cases.pt)"""
     from detectorfreesfm_b200 import refine_stage as rs
-    Ref = ref_shims.import_colmap_dataset_class()
-    a, b, results = _writeback_case(5)
-    Ref.update_refined_kpts_to_colmap_multiview(types.SimpleNamespace(colmap_images=a), results)
+    want = torch.load(CASES_GOLDEN, weights_only=False)["writeback"]
+    _, b, results = _writeback_case(5)
     rs.update_refined_kpts_to_colmap_multiview(b, results)
-    assert all(np.array_equal(a[c].xys, b[c].xys) for c in a)
+    assert set(want) == set(b) and all(np.array_equal(want[c], b[c].xys) for c in b)
