@@ -34,6 +34,7 @@ PROTOTYPES = {
     "dfsfm_coarse_destroy": (None, [c_void_p]),
     "dfsfm_coarse_set_param": (c_int, [c_void_p, c_char_p, c_void_p, c_int64, c_int64, c_int]),
     "dfsfm_coarse_features": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "dfsfm_coarse_features_pair": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dfsfm_coarse_features_fine": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dfsfm_coarse_fine_match": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p,
                                         c_void_p, c_int, c_void_p, c_void_p, c_void_p]),

@@ -102,14 +102,18 @@ class B200LoFTR(torch.nn.Module):
             self._pe[key] = position_encoding(h, w).to(self._device)
         return self._pe[key]
 
+    @staticmethod
+    def _cache_key(image, cache_key):
+        assert image.is_cuda and image.dtype == torch.float32 and image.dim() == 4 and image.shape[0] == 1 and image.shape[1] == 1
+        return None if cache_key is None else (cache_key, image.shape[2], image.shape[3])
+
     def extract_features(self, image, cache_key=None):
         """ResNetFPN_8_2 coarse branch + position encoding -> tokens [(H/8)*(W/8), 256] fp32 (loftr.py:45-59)."""
-        assert image.is_cuda and image.dtype == torch.float32 and image.dim() == 4 and image.shape[0] == 1 and image.shape[1] == 1
-        H, W = image.shape[2:]
-        key = None if cache_key is None else (cache_key, H, W)
+        key = self._cache_key(image, cache_key)
         if key is not None and key in self._cache:
             self._cache.move_to_end(key)
             return self._cache[key]
+        H, W = image.shape[2:]
         image = image.contiguous()
         h, w = H // 8, W // 8
         tokens = torch.empty(h * w, 256, device=self._device, dtype=torch.float32)
@@ -122,14 +126,39 @@ class B200LoFTR(torch.nn.Module):
             _lib.check(self._lib.dfsfm_coarse_features(self._h, _lib.ptr(image), H, W, _lib.ptr(self._pe_tokens(h, w)), _lib.ptr(tokens),
                                                        _lib.stream_ptr(self._device)))
             out = tokens
-        if key is not None:
-            nbytes = sum(t.numel() * t.element_size() for t in (out if isinstance(out, tuple) else (out,)))
-            self._cache[key] = out
-            self._cache_bytes += nbytes
-            while len(self._cache) > 1 and (len(self._cache) > self._cache_size or self._cache_bytes > self._cache_bytes_max):
-                _, old = self._cache.popitem(last=False)
-                self._cache_bytes -= sum(t.numel() * t.element_size() for t in (old if isinstance(old, tuple) else (old,)))
+        self._cache_put(key, out)
         return out
+
+    def extract_features_pair(self, image0, image1, cache_key0=None, cache_key1=None):
+        """``extract_features`` of both images of a pair in one backbone pass (one launch per layer for both) -> (tokens0, tokens1),
+        bitwise equal to two ``extract_features`` calls.  Coarse-only matcher, images of the same size, neither of them cached."""
+        key0, key1 = self._cache_key(image0, cache_key0), self._cache_key(image1, cache_key1)
+        assert self._pair_applies(image0, image1, key0, key1)
+        H, W = image0.shape[2:]
+        image0, image1 = image0.contiguous(), image1.contiguous()
+        h, w = H // 8, W // 8
+        tokens0 = torch.empty(h * w, 256, device=self._device, dtype=torch.float32)
+        tokens1 = torch.empty(h * w, 256, device=self._device, dtype=torch.float32)
+        _lib.check(self._lib.dfsfm_coarse_features_pair(self._h, _lib.ptr(image0), _lib.ptr(image1), H, W, _lib.ptr(self._pe_tokens(h, w)),
+                                                        _lib.ptr(tokens0), _lib.ptr(tokens1), _lib.stream_ptr(self._device)))
+        self._cache_put(key0, tokens0)
+        self._cache_put(key1, tokens1)
+        return tokens0, tokens1
+
+    def _pair_applies(self, image0, image1, key0, key1):
+        # the same name twice is one extraction and one cache entry: the one-image path does that
+        return (not self.fine and image0.shape == image1.shape and (key0 is None or (key0 not in self._cache and key0 != key1))
+                and (key1 is None or key1 not in self._cache))
+
+    def _cache_put(self, key, out):
+        if key is None:
+            return
+        nbytes = sum(t.numel() * t.element_size() for t in (out if isinstance(out, tuple) else (out,)))
+        self._cache[key] = out
+        self._cache_bytes += nbytes
+        while len(self._cache) > 1 and (len(self._cache) > self._cache_size or self._cache_bytes > self._cache_bytes_max):
+            _, old = self._cache.popitem(last=False)
+            self._cache_bytes -= sum(t.numel() * t.element_size() for t in (old if isinstance(old, tuple) else (old,)))
 
     def fine_match(self, feat_f0, hw0_f, feat_f1, hw1_f, feat_c0, hw0_c, feat_c1, hw1_c, i_ids, j_ids):
         """FinePreprocess + loftr_fine + FineMatching -> (coords_normed * (W // 2) [M,2], std [M])."""
@@ -194,8 +223,11 @@ class B200LoFTR(torch.nn.Module):
         if names is not None:
             k0 = names[0][0] if isinstance(names[0], (list, tuple)) else names[0]
             k1 = names[1][0] if isinstance(names[1], (list, tuple)) else names[1]
-        f0 = self.extract_features(im0, k0)
-        f1 = self.extract_features(im1, k1)
+        if self._pair_applies(im0, im1, self._cache_key(im0, k0), self._cache_key(im1, k1)):
+            f0, f1 = self.extract_features_pair(im0, im1, k0, k1)
+        else:
+            f0 = self.extract_features(im0, k0)
+            f1 = self.extract_features(im1, k1)
         if self.fine:
             (f0, ff0), (f1, ff1) = f0, f1
         hw0_c = (im0.shape[2] // 8, im0.shape[3] // 8)

@@ -4,6 +4,7 @@
 #include <algorithm>
 #include <map>
 #include <memory>
+#include <tuple>
 
 #include "../../include/dfsfm_b200.h"
 #include "engine_common.h"
@@ -36,7 +37,7 @@ struct ParityBuf {  // [4 parity][2 hl][rows][C]
     long long plane_stride() const { return 2 * rows * C; }
 };
 
-struct FeatWs {  // backbone workspace for one image geometry
+struct FeatWs {  // backbone workspace for 1 or 2 images of one geometry: every flat buffer holds image 0, then image 1, each with its halo
     Geom g2, g4, g8;
     HL a2, b2, c2;
     ParityBuf p1, p2;
@@ -90,7 +91,8 @@ class CoarseEngine {
     }
     ParamStore params;
 
-    void features(const float* img, int H, int W, const float* pe, float* tokens, float* feat_f, cudaStream_t st);
+    // n_img = 1 or 2 images of the same size in one launch per layer; feat_f (the fine FPN branch) only with one image
+    void features(const float* const* imgs, int n_img, int H, int W, const float* pe, float* const* tokens, float* feat_f, cudaStream_t st);
     void fine_match(const float* ff0, int Hf0, int Wf0, const float* ff1, int Hf1, int Wf1, const float* fc0, int w0c, const float* fc1, int w1c,
                     const int* i_ids, const int* j_ids, int M, float* coords_out, float* std_out, cudaStream_t st);
     void transformer(float* f0, int L, float* f1, int S, cudaStream_t st);
@@ -99,7 +101,7 @@ class CoarseEngine {
 
   private:
     int device_;
-    std::map<std::pair<int, int>, FeatWs> feat_ws_;
+    std::map<std::tuple<int, int, int>, FeatWs> feat_ws_;  // (H, W, n_img)
     TokWs tok_;
     unsigned kv_epoch_ = 0;
     FineWs fine_;
@@ -107,13 +109,14 @@ class CoarseEngine {
     void fine_branch(FeatWs& w, float* feat_f, cudaStream_t st);
     void layer128(int li, bool self, int x0, int xn, int s0, int sn, const Seg* kv_segs, int n_kv, const Seg* apply_segs, int n_apply, cudaStream_t st);
 
-    FeatWs& get_feat_ws(int H, int W);
+    FeatWs& get_feat_ws(int H, int W, int n_img);
     void ensure_tok(int n);
     static void free_feat(FeatWs& w);
     static void free_tok(TokWs& w);
 
     template <int BN>
-    void conv(const HL* ins, int n_in, GemmCore core, const std::string& wname, ConvEpiParams ep, cudaStream_t st);
+    void conv(const HL* ins, int n_in, GemmCore core, const std::string& wname, ConvEpiParams ep, cudaStream_t st, bool allow_slab = true);
+    void conv_l3(int bn, const HL* ins, int n_in, const GemmCore& core, const std::string& wname, const ConvEpiParams& ep, cudaStream_t st);
     void layer_call(int li, bool self, int x0, int xn, int s0, int sn, int kv_seg0, int n_segs, int apply_seg0, int max_count, cudaStream_t st,
                     int seg_row0 = 0);
 };
@@ -173,8 +176,8 @@ static ParityBuf parity_alloc(long long rows, int C) {
     return p;
 }
 
-FeatWs& CoarseEngine::get_feat_ws(int H, int W) {
-    auto key = std::make_pair(H, W);
+FeatWs& CoarseEngine::get_feat_ws(int H, int W, int n_img) {
+    const auto key = std::make_tuple(H, W, n_img);
     auto it = feat_ws_.find(key);
     if (it != feat_ws_.end()) return it->second;
     if (feat_ws_.size() >= 8) {  // bound the cache: drop everything (geometries repeat within a scene)
@@ -185,16 +188,17 @@ FeatWs& CoarseEngine::get_feat_ws(int H, int W) {
     w.g2 = Geom(H / 2, W / 2);
     w.g4 = Geom(H / 4, W / 4);
     w.g8 = Geom(H / 8, W / 8);
-    w.a2 = hl_alloc(w.g2.rows, 128);
-    w.b2 = hl_alloc(w.g2.rows, 128);
-    w.c2 = hl_alloc(w.g2.rows, 128);
-    w.p1 = parity_alloc(w.g4.rows, 128);
-    w.a4 = hl_alloc(w.g4.rows, 208);
-    w.b4 = hl_alloc(w.g4.rows, 208);
-    w.p2 = parity_alloc(w.g8.rows, 208);
-    w.a8 = hl_alloc(w.g8.rows, 256);
-    w.b8 = hl_alloc(w.g8.rows, 256);
-    w.c8 = hl_alloc(w.g8.rows, 256);
+    DFSFM_CHECK(n_img * w.g2.rows < (1ll << 31), "image too large for 32-bit row indices");
+    w.a2 = hl_alloc(n_img * w.g2.rows, 128);
+    w.b2 = hl_alloc(n_img * w.g2.rows, 128);
+    w.c2 = hl_alloc(n_img * w.g2.rows, 128);
+    w.p1 = parity_alloc(n_img * w.g4.rows, 128);
+    w.a4 = hl_alloc(n_img * w.g4.rows, 208);
+    w.b4 = hl_alloc(n_img * w.g4.rows, 208);
+    w.p2 = parity_alloc(n_img * w.g8.rows, 208);
+    w.a8 = hl_alloc(n_img * w.g8.rows, 256);
+    w.b8 = hl_alloc(n_img * w.g8.rows, 256);
+    w.c8 = hl_alloc(n_img * w.g8.rows, 256);
     return feat_ws_.emplace(key, w).first->second;
 }
 void CoarseEngine::free_feat(FeatWs& w) {
@@ -208,9 +212,9 @@ void CoarseEngine::free_feat(FeatWs& w) {
 }
 
 template <int BN>
-void CoarseEngine::conv(const HL* ins, int n_in, GemmCore core, const std::string& wname, ConvEpiParams ep, cudaStream_t st) {
+void CoarseEngine::conv(const HL* ins, int n_in, GemmCore core, const std::string& wname, ConvEpiParams ep, cudaStream_t st, bool allow_slab) {
     const HL& w = params.mat(wname + ".w");
-    const bool slab = BN <= 128 && slab_applicable(core, n_in);
+    const bool slab = BN <= 128 && allow_slab && slab_applicable(core, n_in);
     TmapPack maps;
     for (int i = 0; i < kMaxAMaps; ++i) maps.a[i] = make_tmap(ins[i < n_in ? i : 0], slab ? kSlabRows : kBM);
     maps.b = make_tmap(w, bbox(BN));
@@ -225,6 +229,25 @@ void CoarseEngine::conv(const HL* ins, int n_in, GemmCore core, const std::strin
         }
     }
     launch_gemm_counted<BN, true, ConvEpi>(maps, core, ep, ep.N, st, "conv");
+}
+
+// Column tile width of the 256-channel layer-3 convs: 256, or two 128-wide tiles per row tile when that takes fewer SM-pair rounds
+// counted in half-tile time (a 128-wide tile does half the MMAs of a 256-wide one).  Two 832x832 images: 87 row tiles are 2 full
+// rounds on 74 SM pairs, 174 half tiles are 3 half rounds.  A tie keeps 256 (half the operand traffic per output).
+static int layer3_bn(int M) {
+    const int pairs = sm_count() / 2;
+    const int row_tiles = (M + 2 * kBM - 1) / (2 * kBM);
+    const int full_rounds = (row_tiles + pairs - 1) / pairs;
+    const int half_rounds = (2 * row_tiles + pairs - 1) / pairs;
+    return half_rounds < 2 * full_rounds ? 128 : 256;
+}
+// The 128-wide variant runs without tap slabs: the slab kernel orders a row's K steps kchunk-major within a group of three taps, the
+// plain one tap-major, so only the plain kernel accumulates in the 256-wide kernel's order and the outputs do not depend on the width.
+// (Slabs bought nothing here: 51.7 ms of conv per 28-pair step with or without them, B200 at 1000 W.)
+void CoarseEngine::conv_l3(int bn, const HL* ins, int n_in, const GemmCore& core, const std::string& wname, const ConvEpiParams& ep,
+                           cudaStream_t st) {
+    if (bn == 128) conv<128>(ins, n_in, core, wname, ep, st, false);
+    else conv<256>(ins, n_in, core, wname, ep, st);
 }
 
 static ConvEpiParams epi_flat(const Geom& g, int N, const HL& out, bool relu, const HL* res) {
@@ -247,20 +270,26 @@ static ConvEpiParams epi_parity(const Geom& g, int N, const ParityBuf& out, bool
     return e;
 }
 
-void CoarseEngine::features(const float* img, int H, int W, const float* pe, float* tokens, float* feat_f, cudaStream_t st) {
+// The images of a pair are independent until the transformer, so two images of one size share every launch: each conv runs over the
+// rows of both flat buffers (a tap of an interior output row never leaves its own image's block, and the epilogue maps every row to its
+// image), which gives the launches twice the tiles to spread over the SMs.  Every output row accumulates in the same order as in a
+// one-image call, so the tokens are bitwise the same.
+void CoarseEngine::features(const float* const* imgs, int n_img, int H, int W, const float* pe, float* const* tokens, float* feat_f,
+                            cudaStream_t st) {
     DFSFM_CHECK(H % 8 == 0 && W % 8 == 0 && H >= 16 && W >= 16, "image size must be a multiple of 8 (CoarseMatchingDataset df=8)");
-    FeatWs& w = get_feat_ws(H, W);
+    DFSFM_CHECK(n_img == 1 || (n_img == 2 && !feat_f), "one image, or two without the fine branch");
+    FeatWs& w = get_feat_ws(H, W, n_img);
     // conv1 + bn1 + relu (resnet_fpn.py:102)
     {
-        dim3 grid((w.g2.W + kStemTW - 1) / kStemTW, (w.g2.H + kStemTH - 1) / kStemTH, 1);
+        dim3 grid((w.g2.W + kStemTW - 1) / kStemTW, (w.g2.H + kStemTH - 1) / kStemTH, n_img);
         { LaunchScope ls("stem", st);
-          stem_conv_kernel<<<grid, 128, 0, st>>>(img, H, W, params.vec("stem.w"), params.vec("stem.b"), w.a2.hi, w.a2.lo()); }
+          stem_conv_kernel<<<grid, 128, 0, st>>>(imgs[0], imgs[n_img - 1], H, W, params.vec("stem.w"), params.vec("stem.b"), w.a2.hi, w.a2.lo()); }
         DFSFM_CUDA(cudaGetLastError());
     }
     GemmCore c;
     memset(&c, 0, sizeof(c));
     // layer1 (two BasicBlocks, stride 1, 128 ch) -- resnet_fpn.py:32-40,103
-    c.M = static_cast<int>(w.g2.rows);
+    c.M = static_cast<int>(n_img * w.g2.rows);
     set_k(c, 128);
     conv_taps_s1(c, 3, w.g2.Wp);
     { const HL in[1] = {w.a2}; conv<128>(in, 1, c, "l1.0.c1", epi_flat(w.g2, 128, w.b2, true, nullptr), st); }
@@ -268,7 +297,7 @@ void CoarseEngine::features(const float* img, int H, int W, const float* pe, flo
     { const HL in[1] = {w.c2}; conv<128>(in, 1, c, "l1.1.c1", epi_flat(w.g2, 128, w.b2, true, nullptr), st); }
     { const HL in[1] = {w.b2}; conv<128>(in, 1, c, "l1.1.c2", epi_parity(w.g2, 128, w.p1, true, &w.c2), st); }
     // layer2 (stride 2, 196 -> 208 padded channels) -- the 1x1 stride-2 downsample rides as a 10th tap of conv2
-    c.M = static_cast<int>(w.g4.rows);
+    c.M = static_cast<int>(n_img * w.g4.rows);
     set_k(c, 128);
     conv_taps_s2(c, w.g4.Wp);
     { const HL in[4] = {w.p1.plane(0), w.p1.plane(1), w.p1.plane(2), w.p1.plane(3)};
@@ -281,18 +310,19 @@ void CoarseEngine::features(const float* img, int H, int W, const float* pe, flo
     { const HL in[1] = {w.b4}; conv<208>(in, 1, c, "l2.1.c1", epi_flat(w.g4, 208, w.a4, true, nullptr), st); }
     { const HL in[1] = {w.a4}; conv<208>(in, 1, c, "l2.1.c2", epi_parity(w.g4, 208, w.p2, true, &w.b4), st); }
     // layer3 (stride 2, 256 ch)
-    c.M = static_cast<int>(w.g8.rows);
+    c.M = static_cast<int>(n_img * w.g8.rows);
+    const int bn3 = layer3_bn(c.M);
     set_k(c, 208);
     conv_taps_s2(c, w.g8.Wp);
     { const HL in[4] = {w.p2.plane(0), w.p2.plane(1), w.p2.plane(2), w.p2.plane(3)};
-      conv<256>(in, 4, c, "l3.0.c1", epi_flat(w.g8, 256, w.a8, true, nullptr), st); }
+      conv_l3(bn3, in, 4, c, "l3.0.c1", epi_flat(w.g8, 256, w.a8, true, nullptr), st); }
     set_k(c, 256);
     conv_taps_s1(c, 3, w.g8.Wp);
     c.num_taps = 10; c.tap_map[9] = 1; c.tap_shift[9] = 0;
-    { const HL in[2] = {w.a8, w.p2.plane(0)}; conv<256>(in, 2, c, "l3.0.c2", epi_flat(w.g8, 256, w.b8, true, nullptr), st); }
+    { const HL in[2] = {w.a8, w.p2.plane(0)}; conv_l3(bn3, in, 2, c, "l3.0.c2", epi_flat(w.g8, 256, w.b8, true, nullptr), st); }
     conv_taps_s1(c, 3, w.g8.Wp);
-    { const HL in[1] = {w.b8}; conv<256>(in, 1, c, "l3.1.c1", epi_flat(w.g8, 256, w.a8, true, nullptr), st); }
-    { const HL in[1] = {w.a8}; conv<256>(in, 1, c, "l3.1.c2", epi_flat(w.g8, 256, w.c8, true, &w.b8), st); }
+    { const HL in[1] = {w.b8}; conv_l3(bn3, in, 1, c, "l3.1.c1", epi_flat(w.g8, 256, w.a8, true, nullptr), st); }
+    { const HL in[1] = {w.a8}; conv_l3(bn3, in, 1, c, "l3.1.c2", epi_flat(w.g8, 256, w.c8, true, &w.b8), st); }
     // layer3_outconv (1x1) + position encoding + flatten to tokens (resnet_fpn.py:108, loftr.py:58)
     conv_taps_s1(c, 1, w.g8.Wp);
     {
@@ -302,7 +332,8 @@ void CoarseEngine::features(const float* img, int H, int W, const float* pe, flo
         e.g = w.g8.flat();
         e.addend = pe;
         e.out_mode = OUT_DENSE;
-        e.out_f32 = tokens;
+        e.out_f32 = tokens[0];
+        e.out_f32_1 = n_img == 2 ? tokens[1] : nullptr;
         e.out_f32_ld = 256;
         if (feat_f) {
             if (!w.fine) {
@@ -317,10 +348,10 @@ void CoarseEngine::features(const float* img, int H, int W, const float* pe, flo
             // OUT_DENSE and OUT_FLAT differ only in the row mapping, so the planes come from a second epilogue pass below.
         }
         const HL in[1] = {w.c8};
-        conv<256>(in, 1, c, "out3", e, st);
+        conv_l3(bn3, in, 1, c, "out3", e, st);
         if (feat_f) {
             ConvEpiParams e2 = epi_flat(w.g8, 256, w.x3o, false, nullptr);
-            conv<256>(in, 1, c, "out3", e2, st);
+            conv_l3(bn3, in, 1, c, "out3", e2, st);
             fine_branch(w, feat_f, st);
         }
     }
@@ -942,11 +973,19 @@ int dfsfm_coarse_set_param(dfsfm_coarse_t* h, const char* name, const float* hos
     return dfsfm::guard([&] { h->e->params.set(name, host, rows, cols, kind); });
 }
 int dfsfm_coarse_features(dfsfm_coarse_t* h, const float* image_dev, int H, int W, const float* pe_dev, float* tokens_out_dev, void* stream) {
-    return dfsfm::guard([&] { h->e->features(image_dev, H, W, pe_dev, tokens_out_dev, nullptr, static_cast<cudaStream_t>(stream)); });
+    return dfsfm::guard([&] { h->e->features(&image_dev, 1, H, W, pe_dev, &tokens_out_dev, nullptr, static_cast<cudaStream_t>(stream)); });
+}
+int dfsfm_coarse_features_pair(dfsfm_coarse_t* h, const float* image0_dev, const float* image1_dev, int H, int W, const float* pe_dev,
+                               float* tokens0_out_dev, float* tokens1_out_dev, void* stream) {
+    return dfsfm::guard([&] {
+        const float* imgs[2] = {image0_dev, image1_dev};
+        float* tokens[2] = {tokens0_out_dev, tokens1_out_dev};
+        h->e->features(imgs, 2, H, W, pe_dev, tokens, nullptr, static_cast<cudaStream_t>(stream));
+    });
 }
 int dfsfm_coarse_features_fine(dfsfm_coarse_t* h, const float* image_dev, int H, int W, const float* pe_dev, float* tokens_out_dev,
                                float* feat_f_out_dev, void* stream) {
-    return dfsfm::guard([&] { h->e->features(image_dev, H, W, pe_dev, tokens_out_dev, feat_f_out_dev, static_cast<cudaStream_t>(stream)); });
+    return dfsfm::guard([&] { h->e->features(&image_dev, 1, H, W, pe_dev, &tokens_out_dev, feat_f_out_dev, static_cast<cudaStream_t>(stream)); });
 }
 int dfsfm_coarse_fine_match(dfsfm_coarse_t* h, const float* feat_f0_dev, int Hf0, int Wf0, const float* feat_f1_dev, int Hf1, int Wf1,
                             const float* feat_c0_dev, int w0c, const float* feat_c1_dev, int w1c, const int32_t* i_ids_dev,

@@ -523,6 +523,7 @@ struct ConvEpiParams {
     int out_ld;
     long long plane_stride;  // OUT_PARITY: elements between consecutive parity planes
     float* out_f32;          // optional fp32 copy (same row mapping as out_hi)
+    float* out_f32_1;        // OUT_DENSE: image 1's fp32 rows go here (from row 0) instead of after image 0 in out_f32; may be null
     int out_f32_ld;
     int wy0, wx0, wh, ww;    // OUT_WINDOW / OUT_WINDOW_DENSE
     int ohp, owp;            // OUT_WINDOW / OUT_UNPARITY: rows / pitch of the output geometry
@@ -549,12 +550,18 @@ struct ConvEpi {
         }
         long long orow = row;   // output row index
         long long obase = 0;    // extra element offset (parity plane)
+        float* out_f32 = p.out_f32;
         if (p.out_mode == OUT_PARITY) {
             const int Hp2 = p.g.H / 2 + 1, Wp2 = p.g.W / 2 + 1;
             obase = static_cast<long long>((y & 1) * 2 + (x & 1)) * p.plane_stride;
             orow = static_cast<long long>(n_img) * Hp2 * Wp2 + (y >> 1) * Wp2 + (x >> 1);
         } else if (p.out_mode == OUT_DENSE) {
-            orow = static_cast<long long>(n_img) * p.g.H * p.g.W + y * p.g.W + x;
+            if (n_img == 1 && p.out_f32_1) {
+                out_f32 = p.out_f32_1;
+                orow = y * p.g.W + x;
+            } else {
+                orow = static_cast<long long>(n_img) * p.g.H * p.g.W + y * p.g.W + x;
+            }
         } else if (p.out_mode == OUT_WINDOW) {
             valid = valid && y >= p.wy0 && y < p.wy0 + p.wh && x >= p.wx0 && x < p.wx0 + p.ww;
             orow = static_cast<long long>(n_img) * p.ohp * p.owp + (y - p.wy0) * p.owp + (x - p.wx0);
@@ -643,8 +650,8 @@ struct ConvEpi {
                     }
                 }
             }
-            if (p.out_f32) {
-                float* of = p.out_f32 + orow * p.out_f32_ld + nb;
+            if (out_f32) {
+                float* of = out_f32 + orow * p.out_f32_ld + nb;
 #pragma unroll
                 for (int j = 0; j < 32; j += 4) {
                     if (j < ncnt) *reinterpret_cast<float4*>(of + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);

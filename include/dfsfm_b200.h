@@ -41,6 +41,11 @@ int dfsfm_coarse_set_param(dfsfm_coarse_t* h, const char* name, const float* hos
 int dfsfm_coarse_features(dfsfm_coarse_t* h, const float* image_dev, int H, int W, const float* pe_dev, float* tokens_out_dev,
                           void* stream);
 
+/* Same for the two images of a pair (both H x W) in one launch per layer -- the backbone kernels get twice the tiles to spread
+ * over the SMs.  tokens*_out_dev [(H/8)*(W/8)][256] fp32, bitwise equal to two dfsfm_coarse_features calls. */
+int dfsfm_coarse_features_pair(dfsfm_coarse_t* h, const float* image0_dev, const float* image1_dev, int H, int W, const float* pe_dev,
+                               float* tokens0_out_dev, float* tokens1_out_dev, void* stream);
+
 /* Same, plus the FPN top-down path to the 1/2-resolution fine map x1_out (resnet_fpn.py:110-118, match type 'coarse_fine'):
  * feat_f_out_dev [(H/2)*(W/2)][128] fp32 (NHWC rows). */
 int dfsfm_coarse_features_fine(dfsfm_coarse_t* h, const float* image_dev, int H, int W, const float* pe_dev, float* tokens_out_dev,
